@@ -7,8 +7,9 @@ device, factorization + all inter-GPU traffic + final drain), flop model N^3/3 (
 
   python bench.py --gpus 1 --steps K --warmup W            our arm (N>1: under torchrun, one rank per GPU)
   python bench.py --impl reference --steps K --warmup W    the reference algorithm on the host cores (oracle port)
+  python bench.py ... --dump-outputs DIR                   also write a fixed sample of the last timed factor to DIR/*.npy
 
-One JSON line on stdout (rank 0); everything else goes to stderr.
+One JSON line on stdout (rank 0); everything else goes to stderr. Nothing is written into the source tree.
 """
 from __future__ import annotations
 
@@ -24,10 +25,13 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only; no __pycache__ in it from a benchmark run
 import __graft_entry__ as ge  # noqa: E402
 
 METRIC = "POTRF GFLOP/s (fp64, N=32768, nb=512)"
 GRIDS = {1: (1, 1), 2: (2, 1), 4: (2, 2), 8: (2, 4)}
+DUMP_SAMPLES = 1 << 21  # 16 MB of fp64 (32 MB complex128): the whole factor at N=32768 would be 8 GB
+DUMP_SEED = 20240601
 
 
 def log(*a):
@@ -48,7 +52,7 @@ def parse():
     p.add_argument("--grid-rows", type=int, default=0)
     p.add_argument("--grid-cols", type=int, default=0)
     p.add_argument("--type", default="d", choices=["s", "d", "c", "z"], help="element type (BASELINE metric: d)")
-    p.add_argument("--e2e-steps", type=int, default=-1, help="end-to-end (host buffer) steps, default 5")
+    p.add_argument("--e2e-steps", type=int, default=-1, help="end-to-end (host buffer) steps, default --steps")
     p.add_argument("--parity-n", type=int, default=8192, help="size of the element-wise oracle parity case run after the "
                    "timed region (non-zero source rank on grids; 0 = skip)")
     p.add_argument("--cpu-budget-s", type=float, default=240.0, help="time budget of the CPU arm (whole run)")
@@ -58,7 +62,14 @@ def parse():
     p.add_argument("--next-n", type=int, default=8192, help="size of the short measurements of the algorithms that consume the "
                    "factor (triangular solver, inverse, generalized -> standard; SURVEY 8f), 0 = skip; 1 GPU only")
     p.add_argument("--cpu-sample-n", type=int, default=0, help="force the CPU sample size")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write what the last one computed to DIR/<name>.npy: the factor's diagonal and "
+                        f"{DUMP_SAMPLES} entries of its referenced triangle at positions drawn with a fixed seed (complex types as "
+                        "(..., 2) real/imaginary pairs), so that two builds can be compared output for output")
+    a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    return a
 
 
 # ------------------------------------------------------------------------------------------------
@@ -367,6 +378,34 @@ def triangle_bytes(n: int, nb: int, P: int, Q: int, vr: int, vc: int, itemsize: 
     return total
 
 
+def dump_outputs(out_dir, torch, dist, d_work, n, nb, P, Q, myrow, mycol, ld, rank):
+    """Writes the factor the last timed step left in d_work (this rank's column-major local part, source rank (0, 0)) as
+    DIR/factor_diagonal.npy (all n diagonal entries) and DIR/factor_lower_sample.npy (DUMP_SAMPLES entries (i, j), i >= j,
+    drawn from DUMP_SEED, so the positions depend on n only). Every global entry is owned by exactly one rank: each rank
+    fills the ones it holds into a zero vector and a sum over the ranks assembles the sample on rank 0."""
+    rng = np.random.default_rng(DUMP_SEED)
+    i, j = rng.integers(0, n, DUMP_SAMPLES), rng.integers(0, n, DUMP_SAMPLES)
+    diag = np.arange(n)
+    arrays = {}
+    for name, (rows, cols) in (("factor_diagonal", (diag, diag)),
+                               ("factor_lower_sample", (np.maximum(i, j), np.minimum(i, j)))):
+        mine = ((rows // nb) % P == myrow) & ((cols // nb) % Q == mycol)
+        lrow = (rows // nb) // P * nb + rows % nb
+        lcol = (cols // nb) // Q * nb + cols % nb
+        flat = torch.from_numpy((lcol * ld + lrow)[mine]).cuda()
+        vals = torch.zeros(len(rows), dtype=d_work.dtype, device=d_work.device)
+        vals[torch.from_numpy(mine).cuda()] = d_work.reshape(-1)[flat]
+        if dist is not None:
+            dist.all_reduce(vals)
+        v = vals.cpu().numpy()
+        arrays[name] = np.stack([v.real, v.imag], axis=-1) if np.iscomplexobj(v) else v
+    if rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        for name, v in arrays.items():
+            np.save(os.path.join(out_dir, f"{name}.npy"), v)
+        log(f"[bench] wrote {', '.join(f'{k}.npy {v.shape}' for k, v in arrays.items())} to {out_dir}")
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -461,6 +500,8 @@ def run_ours(args):
     ms_per_step = total_ms / K
     value = flops / (ms_per_step * 1e-3) / 1e9
     clocks = sampler.summary()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, torch, dist if world > 1 else None, d_work, n, nb, P, Q, myrow, mycol, ld, rank)
 
     # ---- correctness of the timed result, for EVERY world size: the product's own distributed result check (the
     # miniapp's check_cholesky on the GPU grid, engine_check.cu: native GEMMs, independent of the int8 engine), and on one
@@ -601,9 +642,9 @@ def run_ours(args):
     })
     del d_work
 
-    # ---- end to end through the reference-facing C ABI with HOST buffers (H2D + D2H inside), E >= 5 steps on pinned
+    # ---- end to end through the reference-facing C ABI with HOST buffers (H2D + D2H inside), E steps on pinned
     # memory plus the same call on PAGEABLE memory (what a ScaLAPACK caller passes)
-    E = args.e2e_steps if args.e2e_steps >= 0 else 5
+    E = args.e2e_steps if args.e2e_steps >= 0 else K
     e2e = None
     if E > 0:
         h_work_t = torch.empty((lc, lr), dtype=tdt, pin_memory=True)
