@@ -7,12 +7,12 @@ CSRC      := dla-future_b200/csrc
 LIBDIR    := dla-future_b200/lib
 LIB       := $(LIBDIR)/libdlaf_b200.so
 
-CU_OBJS  := build/gemm_dmma.o build/gemm_simt.o build/gemm_zdmma.o build/gemm_tf32_tcgen05.o build/gemm_ozaki_i8.o build/potrf_tile.o build/potrf_tile_cluster.o build/layout.o build/engine.o build/sm_partition.o build/peak.o build/engine_check.o build/trsm_engine.o build/inverse_engine.o build/hegst_engine.o
+CU_OBJS  := build/gemm_dmma.o build/gemm_simt.o build/gemm_zdmma.o build/gemm_tf32_tcgen05.o build/gemm_ozaki_i8.o build/potrf_tile.o build/potrf_tile_cluster.o build/layout.o build/engine.o build/sm_partition.o build/peak.o build/engine_check.o build/trsm_engine.o build/trmm_engine.o build/inverse_engine.o build/hegst_engine.o
 CPP_OBJS := build/comm.o build/c_api.o build/util_matrix.o build/pool.o
 OBJS     := $(CU_OBJS) $(CPP_OBJS)
 HDRS     := $(wildcard $(CSRC)/*.cuh) $(wildcard $(CSRC)/*.h) $(wildcard include/dlaf_c/*.h) $(wildcard include/dlaf_c/factorization/*.h) $(wildcard include/dlaf_c/inverse/*.h)
 
-all: $(LIB) tools/gpu_diag_tile_test tools/gpu_kernel_test tools/gpu_chain_test tools/gpu_ozaki_test tools/cusolver_potrf_ref tools/cublas_tile_potrf_ref tools/cusolvermg_potrf_ref miniapp/miniapp_cholesky
+all: $(LIB) tools/gpu_diag_tile_test tools/gpu_kernel_test tools/gpu_chain_test tools/gpu_ozaki_test tools/cusolver_potrf_ref tools/cublas_tile_potrf_ref tools/cusolvermg_potrf_ref tools/cublas_trmm_ref miniapp/miniapp_cholesky
 
 build/%.o: $(CSRC)/%.cu $(HDRS)
 	@mkdir -p build
@@ -50,12 +50,15 @@ tools/cublas_tile_potrf_ref: tools/cublas_tile_potrf_ref.cu
 tools/cusolvermg_potrf_ref: tools/cusolvermg_potrf_ref.cu
 	$(NVCC) $(NVCCFLAGS) $< -lcusolverMg -lcusolver -lcublas -o $@
 
+tools/cublas_trmm_ref: tools/cublas_trmm_ref.cu
+	$(NVCC) $(NVCCFLAGS) $< -lcublas -o $@
+
 # The driver is plain C++ against include/dlaf (header-only surface) + the C-ABI library.
 miniapp/miniapp_cholesky: miniapp/miniapp_cholesky.cpp $(LIB) $(wildcard include/dlaf/*.h) $(wildcard include/dlaf/*/*.h)
 	g++ $(CXXFLAGS) $< -o $@ -L$(LIBDIR) -ldlaf_b200 -L/usr/local/cuda/lib64 -lcudart -Wl,-rpath,'$$ORIGIN/../$(LIBDIR)' -Wl,-rpath,/usr/local/cuda/lib64 -lpthread
 
 clean:
 	rm -rf build tools/gpu_diag_tile_test tools/gpu_kernel_test tools/gpu_chain_test tools/gpu_ozaki_test tools/cusolver_potrf_ref \
-	       tools/cublas_tile_potrf_ref tools/cusolvermg_potrf_ref miniapp/miniapp_cholesky $(LIBDIR)/*.so
+	       tools/cublas_tile_potrf_ref tools/cusolvermg_potrf_ref tools/cublas_trmm_ref miniapp/miniapp_cholesky $(LIBDIR)/*.so
 
 .PHONY: all clean

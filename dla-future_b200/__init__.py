@@ -39,6 +39,7 @@ C_API_SYMBOLS = [
     "dlaf_b200_set_profiling", "dlaf_b200_read_profile", "dlaf_b200_read_chain_profile", "dlaf_b200_measure_fp64_tensor_peak_tflops", "dlaf_b200_measure_int8_tensor_peak_tops",
     "dlaf_b200_local_rows", "dlaf_b200_local_cols",
     *[f"dlaf_b200_triangular_solver_{t}" for t in "sdcz"], "dlaf_b200_last_solver_launch_count", "dlaf_b200_last_solver_device_ms",
+    *[f"dlaf_b200_triangular_multiplication_{t}" for t in "sdcz"], *[f"dlaf_b200_triangular_multiplication_device_{t}" for t in "sdcz"],
     *[f"dlaf_inverse_from_cholesky_factor_{t}" for t in "sdcz"], *[f"dlaf_p{t}potri" for t in "sdcz"],
     *[f"dlaf_b200_triangular_inverse_{t}" for t in "sdcz"], *[f"dlaf_b200_assemble_cholesky_inverse_{t}" for t in "sdcz"],
     *[f"dlaf_b200_inverse_device_{t}" for t in "sdcz"], "dlaf_b200_last_inverse_guard_steps",
@@ -142,6 +143,12 @@ def lib() -> ctypes.CDLL:
         f.restype = ctypes.c_double
         f = getattr(L, f"dlaf_b200_triangular_solver_{t}")
         f.argtypes = [ci, cc, cc, cc, cc, vp, vp, DLAF_descriptor, vp, DLAF_descriptor]
+        f.restype = ci
+        f = getattr(L, f"dlaf_b200_triangular_multiplication_{t}")
+        f.argtypes = [ci, cc, cc, cc, cc, vp, vp, DLAF_descriptor, vp, DLAF_descriptor]
+        f.restype = ci
+        f = getattr(L, f"dlaf_b200_triangular_multiplication_device_{t}")
+        f.argtypes = [ci, cc, cc, cc, cc, vp, vp, DLAF_descriptor, vp, DLAF_descriptor, vp]
         f.restype = ci
         f = getattr(L, f"dlaf_b200_check_cholesky_device_{t}")
         f.argtypes = [ci, cc, vp, vp, DLAF_descriptor, vp]
@@ -332,6 +339,36 @@ def triangular_solver(ctx: int, side: str, uplo: str, op: str, diag: str, alpha,
     al = np.array([alpha], dtype=b.dtype)
     f = getattr(lib(), f"dlaf_b200_triangular_solver_{type_char(b.dtype)}")
     f(ctx, side.encode(), uplo.encode(), op.encode(), diag.encode(), al.ctypes.data, a.ctypes.data, da, b.ctypes.data, db)
+
+
+def _triangular_descriptors(side: str, m: int, n: int, mb: int, nb: int, lda: int, ldb: int, isrc: int, jsrc: int):
+    na, ba = (m, mb) if side.upper() == "L" else (n, nb)
+    return (DLAF_descriptor(na, na, ba, ba, isrc, jsrc, 0, 0, max(1, lda)),
+            DLAF_descriptor(m, n, mb, nb, isrc, jsrc, 0, 0, max(1, ldb)))
+
+
+def triangular_multiplication(ctx: int, side: str, uplo: str, op: str, diag: str, alpha, a: np.ndarray, b: np.ndarray, mb: int,
+                              nb: int, m: int | None = None, n: int | None = None, isrc: int = 0, jsrc: int = 0) -> None:
+    """dlaf::triangular_multiplication through the C ABI: B <- alpha op(A) B (side 'L') or B <- alpha B op(A) (side 'R');
+    arguments as for `triangular_solver`, `b` is overwritten with the product."""
+    if a.dtype != b.dtype:
+        raise TypeError(f"A ({a.dtype}) and B ({b.dtype}) must have the same element type")
+    m = b.shape[0] if m is None else m
+    n = b.shape[1] if n is None else n
+    da, db = _triangular_descriptors(side, m, n, mb, nb, _ld_of(a), _ld_of(b), isrc, jsrc)
+    al = np.array([alpha], dtype=b.dtype)
+    f = getattr(lib(), f"dlaf_b200_triangular_multiplication_{type_char(b.dtype)}")
+    f(ctx, side.encode(), uplo.encode(), op.encode(), diag.encode(), al.ctypes.data, a.ctypes.data, da, b.ctypes.data, db)
+
+
+def triangular_multiplication_device(ctx: int, side: str, uplo: str, op: str, diag: str, alpha, a_dev: int, b_dev: int, dtype,
+                                     m: int, n: int, mb: int, nb: int, lda: int, ldb: int, stream: int = 0, isrc: int = 0,
+                                     jsrc: int = 0) -> int:
+    """The triangular multiplication on DEVICE local parts (column-major, leading dimensions lda / ldb); synchronous."""
+    da, db = _triangular_descriptors(side, m, n, mb, nb, lda, ldb, isrc, jsrc)
+    al = np.array([alpha], dtype=dtype)
+    f = getattr(lib(), f"dlaf_b200_triangular_multiplication_device_{type_char(dtype)}")
+    return f(ctx, side.encode(), uplo.encode(), op.encode(), diag.encode(), al.ctypes.data, a_dev, da, b_dev, db, stream)
 
 
 def inverse_from_cholesky_factor(ctx: int, uplo: str, a: np.ndarray, nb: int, n: int | None = None, isrc: int = 0,

@@ -1,6 +1,8 @@
-// Kernels and host helpers shared by the triangular solver (trsm_engine.cu) and the inverse engine (inverse_engine.cu):
-// tile packing with transposition / conjugation / negation, inverses of the G x G diagonal blocks of triangular tiles,
-// the block substitution  Y <- Y G^-H  against one triangular tile, local tile counting.
+// Kernels and host helpers shared by the triangular solver (trsm_engine.cu), the triangular multiplication
+// (trmm_engine.cu) and the inverse engine (inverse_engine.cu): the load of the triangular matrix and the B <-> Y
+// conversion of the two triangular sweeps (tri_sweep.cuh), tile packing with transposition / conjugation / negation,
+// inverses of the G x G diagonal blocks of triangular tiles, the block substitution  Y <- Y G^-H  against one triangular
+// tile, local tile counting.
 #pragma once
 
 #include <cuda_runtime.h>
@@ -263,6 +265,70 @@ __global__ void inv_convert_kernel(T* __restrict__ a, long lda, T* __restrict__ 
         else
           a[(ur0 + r) + (uc0 + c) * lda] = t[k][tx];
       }
+    }
+  }
+}
+
+// Caller's local part of the triangular matrix -> padded tiles (nbp x nbp, ld = ltr * nbp): only the referenced triangle
+// is taken (the other one may hold anything), diagonal tiles get zeros in their unreferenced half, the padding of
+// diagonal tiles an identity, Diag::Unit puts ones on the diagonal. One CTA per (tile, column).
+template <class T>
+__global__ void trsm_load_a_kernel(const T* __restrict__ a, long lda, T* __restrict__ slab, long lds, long na, int ba, int nbp,
+                                   int P, int Q, int prow, int pcol, int ltr, bool lower, bool unit) {
+  const int tile = blockIdx.x, s = blockIdx.y;
+  const int la = tile % ltr, lb = tile / ltr;
+  const long ga = static_cast<long>(la) * P + prow, gb = static_cast<long>(lb) * Q + pcol;
+  const int rows = static_cast<int>(min(static_cast<long>(ba), na - ga * ba));
+  const int cols = static_cast<int>(min(static_cast<long>(ba), na - gb * ba));
+  T* dst = slab + static_cast<long>(la) * nbp + (static_cast<long>(lb) * nbp + s) * lds;
+  const T* src = a + static_cast<long>(la) * ba + (static_cast<long>(lb) * ba + s) * lda;
+  const bool tile_ref = (ga == gb) || (lower ? ga > gb : ga < gb);
+  for (int r = threadIdx.x; r < nbp; r += blockDim.x) {
+    const bool in = r < rows && s < cols;
+    T v = make_real<T>(0);
+    if (ga == gb) {
+      if (r == s)
+        v = (in && !unit) ? src[r] : make_real<T>(1);
+      else if (lower ? r > s : r < s)
+        v = in ? src[r] : make_real<T>(0);
+    }
+    else if (tile_ref && in) {
+      v = src[r];
+    }
+    dst[r] = v;
+  }
+}
+
+// Y <- c * B (Right: same orientation) or c * B^H (Left), B = caller's local part (lrb x lcb valid, ldb), Y = slab with
+// ldy rows; Y's columns are tiles of `by` user columns padded to nbp. transposed: Y(r, tile(c)) = conj(B(c, r)).
+//   not transposed: Y rows = B rows (contiguous), Y col tiles = B col tiles (block by -> nbp)
+//   transposed    : Y rows = B cols (contiguous), Y col tiles = B row tiles (block by -> nbp)
+template <class T, bool TO_Y>
+__global__ void trsm_convert_y_kernel(T* __restrict__ b, long ldb, long lrb, long lcb, T* __restrict__ y, long ldy, int by,
+                                      int nbp, bool transposed, double cre, double cim) {
+  // blockIdx.x = column of Y (padded index), threads over rows of Y
+  const long yc = blockIdx.x;
+  const long tile = yc / nbp, off = yc % nbp;
+  const long uc = tile * by + off;  // index along the tiled user dimension
+  const bool col_ok = off < by;
+  const long nrows_y = transposed ? lcb : lrb;
+  const long ntiled = transposed ? lrb : lcb;
+  for (long r = threadIdx.x + static_cast<long>(blockIdx.y) * blockDim.x; r < ldy; r += static_cast<long>(blockDim.x) * gridDim.y) {
+    const bool in = col_ok && uc < ntiled && r < nrows_y;
+    if (TO_Y) {
+      T v = make_real<T>(0);
+      if (in) {
+        const T u = transposed ? conj_val(b[uc + r * ldb]) : b[r + uc * ldb];
+        v = scale_c(u, cre, cim);
+      }
+      y[r + yc * ldy] = v;
+    }
+    else if (in) {
+      const T v = y[r + yc * ldy];
+      if (transposed)
+        b[uc + r * ldb] = conj_val(v);
+      else
+        b[r + uc * ldb] = v;
     }
   }
 }

@@ -11,186 +11,39 @@
 #include "distribution.h"
 #include "gemm_ozaki.h"
 #include "pool.h"
-#include "tri_kernels.cuh"
+#include "tri_sweep.cuh"
 
 namespace dlaf_b200 {
 
-namespace {
-
 using namespace trik;
-
-// Caller's local part of the triangular matrix -> padded tiles (nbp x nbp, ld = ltr * nbp): only the referenced triangle
-// is taken (the other one may hold anything), diagonal tiles get zeros in their unreferenced half, the padding of
-// diagonal tiles an identity, Diag::Unit puts ones on the diagonal. One CTA per (tile, column).
-template <class T>
-__global__ void trsm_load_a_kernel(const T* __restrict__ a, long lda, T* __restrict__ slab, long lds, long na, int ba, int nbp,
-                                   int P, int Q, int prow, int pcol, int ltr, bool lower, bool unit) {
-  const int tile = blockIdx.x, s = blockIdx.y;
-  const int la = tile % ltr, lb = tile / ltr;
-  const long ga = static_cast<long>(la) * P + prow, gb = static_cast<long>(lb) * Q + pcol;
-  const int rows = static_cast<int>(min(static_cast<long>(ba), na - ga * ba));
-  const int cols = static_cast<int>(min(static_cast<long>(ba), na - gb * ba));
-  T* dst = slab + static_cast<long>(la) * nbp + (static_cast<long>(lb) * nbp + s) * lds;
-  const T* src = a + static_cast<long>(la) * ba + (static_cast<long>(lb) * ba + s) * lda;
-  const bool tile_ref = (ga == gb) || (lower ? ga > gb : ga < gb);
-  for (int r = threadIdx.x; r < nbp; r += blockDim.x) {
-    const bool in = r < rows && s < cols;
-    T v = make_real<T>(0);
-    if (ga == gb) {
-      if (r == s)
-        v = (in && !unit) ? src[r] : make_real<T>(1);
-      else if (lower ? r > s : r < s)
-        v = in ? src[r] : make_real<T>(0);
-    }
-    else if (tile_ref && in) {
-      v = src[r];
-    }
-    dst[r] = v;
-  }
-}
-
-// Y <- c * B (Right: same orientation) or c * B^H (Left), B = caller's local part (lrb x lcb valid, ldb), Y = slab with
-// ldy rows; Y's columns are tiles of `by` user columns padded to nbp. transposed: Y(r, tile(c)) = conj(B(c, r)).
-//   not transposed: Y rows = B rows (contiguous), Y col tiles = B col tiles (block by -> nbp)
-//   transposed    : Y rows = B cols (contiguous), Y col tiles = B row tiles (block by -> nbp)
-template <class T, bool TO_Y>
-__global__ void trsm_convert_y_kernel(T* __restrict__ b, long ldb, long lrb, long lcb, T* __restrict__ y, long ldy, int by,
-                                      int nbp, bool transposed, double cre, double cim) {
-  // blockIdx.x = column of Y (padded index), threads over rows of Y
-  const long yc = blockIdx.x;
-  const long tile = yc / nbp, off = yc % nbp;
-  const long uc = tile * by + off;  // index along the tiled user dimension
-  const bool col_ok = off < by;
-  const long nrows_y = transposed ? lcb : lrb;
-  const long ntiled = transposed ? lrb : lcb;
-  for (long r = threadIdx.x + static_cast<long>(blockIdx.y) * blockDim.x; r < ldy; r += static_cast<long>(blockDim.x) * gridDim.y) {
-    const bool in = col_ok && uc < ntiled && r < nrows_y;
-    if (TO_Y) {
-      T v = make_real<T>(0);
-      if (in) {
-        const T u = transposed ? conj_val(b[uc + r * ldb]) : b[r + uc * ldb];
-        v = scale_c(u, cre, cim);
-      }
-      y[r + yc * ldy] = v;
-    }
-    else if (in) {
-      const T v = y[r + yc * ldy];
-      if (transposed)
-        b[uc + r * ldb] = conj_val(v);
-      else
-        b[r + uc * ldb] = v;
-    }
-  }
-}
-
-}  // namespace
 
 template <class T>
 long triangular_solve_device(const TrsmProblem& p, double alpha_re, double alpha_im, const T* a_user, long lda, T* b_user,
                              long ldb, ncclComm_t row_comm, ncclComm_t col_comm, cudaStream_t s) {
-  using NT = NcclType<T>;
   constexpr int G = Gran<T>::value;
-  long launches = 0;
-  const bool left = (p.side == 'L' || p.side == 'l');
-  const bool a_lower = (p.uplo == 'L' || p.uplo == 'l');
-  const char opc = (p.op == 'n') ? 'N' : ((p.op == 't') ? 'T' : ((p.op == 'c') ? 'C' : p.op));
-  DLAF_B200_ASSERT(opc == 'N' || opc == 'T' || opc == 'C', "op must be N, T or C");
-  const bool unit = (p.diag == 'U' || p.diag == 'u');
-  const bool is_complex = sizeof(T) == 2 * sizeof(base_t<T>);
-  // G = M^H: Left: op(A); Right: op(A)^H
-  const bool tr = left ? (opc != 'N') : (opc == 'N');
-  const bool cj = is_complex && (left ? (opc == 'C') : (opc != 'C'));
-  const bool g_lower = a_lower != tr;
-  const bool forward = g_lower;
-  const double cre = alpha_re, cim = left ? -alpha_im : alpha_im;  // c = conj(alpha) (Left) / alpha (Right)
-
-  const long na = left ? p.m : p.n;
-  const int ba = left ? p.mb : p.nb;
-  if (na == 0 || p.m == 0 || p.n == 0)
+  TriSweep<T> sw;
+  // every packed diagonal tile is followed by the inverses of its ns G x G blocks: [tile | W], W = nbp * G elements
+  const size_t wsz = static_cast<size_t>(round_up(p.side == 'L' || p.side == 'l' ? p.mb : p.nb, G)) * G;
+  if (!sw.setup(p, alpha_re, alpha_im, a_user, lda, b_user, ldb, row_comm, col_comm, s, wsz))
     return 0;
-  const int nbp = static_cast<int>(round_up(ba, G));
-  const int ns = nbp / G;
-  const int nt = ceil_div(na, ba);
-  const size_t tsz = static_cast<size_t>(nbp) * nbp, wsz = static_cast<size_t>(ns) * G * G;
-  const int P = p.P, Q = p.Q;
-  // ---- engine grid (roles swapped for Side::Left: the engine works on Y = B^H)
-  const int Pe = left ? Q : P, Qe = left ? P : Q;
-  const int erow = left ? p.pcol : p.prow, ecol = left ? p.prow : p.pcol;
-  ncclComm_t e_row_comm = left ? col_comm : row_comm;  // ranks of my ENGINE row (size Qe)
-  ncclComm_t e_col_comm = left ? row_comm : col_comm;  // ranks of my ENGINE column (size Pe)
-  const int e_src_in_col = left ? p.src_col : p.src_row, e_src_in_row = left ? p.src_row : p.src_col;
-  auto col_rank = [&](int v_erow) { return (v_erow + e_src_in_col) % Pe; };
-  auto row_rank = [&](int v_ecol) { return (v_ecol + e_src_in_row) % Qe; };
-  DLAF_B200_ASSERT(Pe == 1 || e_col_comm != nullptr, "communicator required");
-  DLAF_B200_ASSERT(Qe == 1 || e_row_comm != nullptr, "communicator required");
-  // where the stored tile of G(t, k) sits, in ENGINE coordinates: pattern N = (t % Pe, k % Qe), pattern T = (k % Pe, t % Qe)
-  const bool pattern_n = (left == tr);
-
-  // ---- the triangular matrix: my local tiles, padded
-  const int ltrA = cnt(nt, p.prow, P), ltcA = cnt(nt, p.pcol, Q);
-  T* a_slab = nullptr;
-  const long lds = static_cast<long>(ltrA > 0 ? ltrA : 1) * nbp;
-  if (ltrA > 0 && ltcA > 0) {
-    a_slab = pool_alloc<T>(lds * ltcA * nbp);
-    dim3 grid(ltrA * ltcA, nbp);
-    trsm_load_a_kernel<T><<<grid, 128, 0, s>>>(a_user, lda, a_slab, lds, na, ba, nbp, P, Q, p.prow, p.pcol, ltrA, a_lower, unit);
-    DLAF_CUDA_CHECK(cudaGetLastError());
-    ++launches;
-  }
-  auto a_tile = [&](long ga, long gb) { return a_slab + (ga / P) * nbp + (gb / Q) * nbp * lds; };  // local stored tile (ga, gb)
-  auto pack = [&](const T* src, T* dst, int ntiles, long src_stride, long dst_stride) {
-    if (ntiles <= 0)
-      return;
-    dim3 grid(nbp / 32, nbp / 32, ntiles), block(32, 8);
-    trsm_pack_tile_kernel<T><<<grid, block, 0, s>>>(src, lds, dst, nbp, tr, cj, src_stride, dst_stride, nbp, false);
-    DLAF_CUDA_CHECK(cudaGetLastError());
-    ++launches;
-  };
-
-  // ---- Y: local rows (contiguous, padded to 128) x my block columns (tiles of ba -> nbp)
-  const long lrb = local_size_1d(p.m, p.mb, P, p.prow), lcb = local_size_1d(p.n, p.nb, Q, p.pcol);
-  const long yrows = left ? lcb : lrb;
-  const long ldy = round_up(yrows > 0 ? yrows : 1, 128);
-  const int ltcY = cnt(nt, ecol, Qe);
-  T* y = nullptr;
-  if (ltcY > 0) {
-    y = pool_alloc<T>(ldy * ltcY * nbp);
-    dim3 grid(static_cast<unsigned>(ltcY * nbp), static_cast<unsigned>((ldy + 1023) / 1024 > 0 ? (ldy + 1023) / 1024 : 1));
-    trsm_convert_y_kernel<T, true><<<grid, 256, 0, s>>>(b_user, ldb, lrb, lcb, y, ldy, ba, nbp, left, cre, cim);
-    DLAF_CUDA_CHECK(cudaGetLastError());
-    ++launches;
-  }
-
-  // ---- my diagonal tiles of G, packed, + the inverses of their GB-blocks: [tile | W] per local diagonal tile
-  std::vector<int> my_diag;  // global k of the diagonal tiles I own
-  for (int k = 0; k < nt; ++k)
-    if (k % P == p.prow && k % Q == p.pcol)
-      my_diag.push_back(k);
-  T* dloc = nullptr;
-  if (!my_diag.empty()) {
-    dloc = pool_alloc<T>((tsz + wsz) * my_diag.size());
-    for (size_t i = 0; i < my_diag.size(); ++i)
-      pack(a_tile(my_diag[i], my_diag[i]), dloc + (tsz + wsz) * i, 1, 0, 0);
-    dim3 grid(ns, static_cast<unsigned>(my_diag.size()));
+  const int nbp = sw.nbp, ns = sw.ns, nt = sw.nt, Pe = sw.Pe, Qe = sw.Qe, ecol = sw.ecol, ltcY = sw.ltcY;
+  const long ldy = sw.ldy;
+  const size_t tsz = sw.tsz;
+  const bool g_lower = sw.g_lower, forward = g_lower, pattern_n = sw.pattern_n;
+  T* y = sw.y;
+  if (!sw.my_diag.empty()) {
+    dim3 grid(ns, static_cast<unsigned>(sw.my_diag.size()));
     static bool configured = false;
     if (!configured) {
       DLAF_CUDA_CHECK(cudaFuncSetAttribute(trsm_trtri_blocks_kernel<T, G>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                            static_cast<int>(sizeof(T) * G * (G + 1))));
       configured = true;
     }
-    trsm_trtri_blocks_kernel<T, G><<<grid, G, sizeof(T) * G * (G + 1), s>>>(dloc, static_cast<long>(tsz + wsz), nbp, dloc + tsz,
-                                                                           static_cast<long>(tsz + wsz), g_lower);
+    trsm_trtri_blocks_kernel<T, G><<<grid, G, sizeof(T) * G * (G + 1), s>>>(sw.dloc, static_cast<long>(sw.dsz), nbp, sw.dloc + tsz,
+                                                                           static_cast<long>(sw.dsz), g_lower);
     DLAF_CUDA_CHECK(cudaGetLastError());
-    ++launches;
+    ++sw.launches;
   }
-  // ---- workspaces of the sweep
-  T *dbuf = nullptr, *panelY = nullptr, *panelR = nullptr, *panelG = nullptr;
-  dbuf = pool_alloc<T>((tsz + wsz));
-  panelY = pool_alloc<T>(ldy * nbp);
-  const int ltrR = cnt(nt, erow, Pe);  // tiles t with t % Pe == erow (pattern N: what arrives along my engine row)
-  if (pattern_n)
-    panelR = pool_alloc<T>(tsz * (ltrR > 0 ? ltrR : 1));
-  panelG = pool_alloc<T>(tsz * (ltcY > 0 ? ltcY : 1));
 
   // fp64: the per-step update runs on tcgen05 as exact int8 digit products (gemm_ozaki.h), like the POTRF trailing update —
   // Y_k and the G tiles of the step are cut into digit planes first; same guard (a step whose operands span too many
@@ -203,7 +56,7 @@ long triangular_solve_device(const TrsmProblem& p, double alpha_re, double alpha
     use_oz = (e == nullptr || std::string(e) == "ozaki") && nbp <= 512 && ltcY > 0 && nt > 1;
     if (use_oz) {
       oz_a.allocate(ldy, nbp);
-      oz_b.allocate(static_cast<long>(pattern_n && Pe == 1 ? (ltrR > 0 ? ltrR : 1) : ltcY) * nbp, nbp);
+      oz_b.allocate(static_cast<long>(pattern_n && Pe == 1 ? (sw.ltrR > 0 ? sw.ltrR : 1) : ltcY) * nbp, nbp);
       oz_flag = pool_alloc<int>(nt);
       DLAF_CUDA_CHECK(cudaMemsetAsync(oz_flag, 0, sizeof(int) * nt, s));
     }
@@ -212,115 +65,26 @@ long triangular_solve_device(const TrsmProblem& p, double alpha_re, double alpha
     if (g.M <= 0 || g.N <= 0 || g.K <= 0)
       return;
     launch_gemm_nt<T>(g, s);
-    ++launches;
-  };
-  // Y_k <- Y_k Gkk^-H by block substitution over the GB-blocks of the tile (tri_kernels.cuh)
-  auto solve_tile = [&](T* yk, const T* gkk, const T* w) {
-    launches += solve_rows_against_tile<T>(yk, ldy, ldy, gkk, nbp, w, ns, g_lower, s);
+    ++sw.launches;
   };
 
   // ---- the sweep
   for (int step = 0; step < nt; ++step) {
     const int k = forward ? step : nt - 1 - step;
-    const int owner_r = k % Pe, owner_c = k % Qe;
-    const bool in_col = (ecol == owner_c);
-    // remaining block columns t: (k, nt) forward, [0, k) backward
-    const int lj0 = forward ? cnt(k + 1, ecol, Qe) : 0;                 // my local Y columns in the remaining set
-    const int lj1 = forward ? ltcY : cnt(k, ecol, Qe);
-    const int li0 = forward ? cnt(k + 1, erow, Pe) : 0;                 // row-index tiles t % Pe == erow in the remaining set
-    const int li1 = forward ? ltrR : cnt(k, erow, Pe);
-    const bool more = forward ? (k < nt - 1) : (k > 0);
-
-    // (1) diagonal tile + inverted blocks down the engine column that holds Y_k
-    const T* gkk = nullptr;
-    const T* w = nullptr;
-    if (in_col) {
-      const bool i_own = (erow == owner_r);
-      const T* mine = nullptr;
-      if (i_own) {
-        size_t idx = 0;
-        while (my_diag[idx] != k)
-          ++idx;
-        mine = dloc + (tsz + wsz) * idx;
-      }
-      if (Pe > 1) {
-        DLAF_NCCL_CHECK(ncclBroadcast(i_own ? mine : dbuf, dbuf, (tsz + wsz) * NT::mult, NT::value, col_rank(owner_r), e_col_comm, s));
-        gkk = dbuf;
-      }
-      else {
-        gkk = mine;
-      }
-      w = gkk + tsz;
-      // (2) my rows of Y_k
-      solve_tile(y + static_cast<long>(k / Qe) * nbp * ldy, gkk, w);
+    const auto st = sw.step(k);
+    // (1) diagonal tile + inverted blocks down the engine column that holds Y_k, (2) my rows of Y_k <- Y_k Gkk^-H by block
+    // substitution over the G-blocks of the tile (tri_kernels.cuh)
+    if (st.in_col) {
+      const T* gkk = sw.diag(st);
+      sw.launches += solve_rows_against_tile<T>(sw.y_col(k), ldy, ldy, gkk, nbp, gkk + tsz, ns, g_lower, s);
     }
-    if (!more)
+    if (!st.more)
       break;
-    // (3) the solved block column along the engine rows
-    const T* ya = nullptr;
-    if (Qe > 1) {
-      const T* send = in_col ? y + static_cast<long>(k / Qe) * nbp * ldy : panelY;
-      DLAF_NCCL_CHECK(ncclBroadcast(send, panelY, static_cast<size_t>(ldy) * nbp * NT::mult, NT::value, row_rank(owner_c), e_row_comm, s));
-      ya = panelY;
-    }
-    else {
-      ya = y + static_cast<long>(k / Qe) * nbp * ldy;
-    }
-    // (4) the tiles G(t, k) for my remaining block columns t
-    const T* gb = nullptr;
-    long b_ts = static_cast<long>(tsz);
-    const int ncols = lj1 - lj0;
-    if (pattern_n) {
-      // stored tile of G(t, k) sits at engine (t % Pe, k % Qe): along the row first, then down the columns
-      const int nrow_tiles = li1 - li0;
-      if (nrow_tiles > 0) {
-        if (in_col) {
-          // my tiles t = (li0 + i) * Pe + erow, i < nrow_tiles; stored (a, b) = (t, k) [Right] or (k, t) [Left]
-          const long t0 = static_cast<long>(li0) * Pe + erow;
-          const T* src = left ? a_tile(k, t0) : a_tile(t0, k);
-          const long stride = left ? static_cast<long>(nbp) * lds : static_cast<long>(nbp);  // next t: next local column / row of A
-          pack(src, panelR, nrow_tiles, stride, static_cast<long>(tsz));
-        }
-        if (Qe > 1)
-          DLAF_NCCL_CHECK(ncclBroadcast(panelR, panelR, tsz * nrow_tiles * NT::mult, NT::value, row_rank(owner_c), e_row_comm, s));
-      }
-      if (Pe > 1) {
-        if (ncols > 0) {
-          DLAF_NCCL_CHECK(ncclGroupStart());
-          for (int lj = lj0; lj < lj1; ++lj) {
-            const long t = static_cast<long>(lj) * Qe + ecol;
-            const int root_v = static_cast<int>(t % Pe);
-            T* recv = panelG + tsz * (lj - lj0);
-            const T* send = recv;
-            if (root_v == erow)
-              send = panelR + tsz * (t / Pe - li0);
-            DLAF_NCCL_CHECK(ncclBroadcast(send, recv, tsz * NT::mult, NT::value, col_rank(root_v), e_col_comm, s));
-          }
-          DLAF_NCCL_CHECK(ncclGroupEnd());
-        }
-        gb = panelG;
-      }
-      else {
-        // one engine row: every remaining tile arrived along the row; my block columns are every Qe-th of them
-        const long t_first = static_cast<long>(lj0) * Qe + ecol;
-        gb = panelR + tsz * (t_first - (forward ? k + 1 : 0));
-        b_ts = static_cast<long>(tsz) * Qe;
-      }
-    }
-    else {
-      // stored tile of G(t, k) sits at engine (k % Pe, t % Qe): already in my engine column -> straight down it
-      if (ncols > 0) {
-        if (erow == owner_r) {
-          const long t0 = static_cast<long>(lj0) * Qe + ecol;
-          const T* src = left ? a_tile(t0, k) : a_tile(k, t0);  // stored (a, b) = (t, k) [Left] or (k, t) [Right]
-          const long stride = left ? static_cast<long>(nbp) : static_cast<long>(nbp) * lds;
-          pack(src, panelG, ncols, stride, static_cast<long>(tsz));
-        }
-        if (Pe > 1)
-          DLAF_NCCL_CHECK(ncclBroadcast(panelG, panelG, tsz * ncols * NT::mult, NT::value, col_rank(owner_r), e_col_comm, s));
-      }
-      gb = panelG;
-    }
+    // (3) the solved block column along the engine rows, (4) the tiles G(t, k) for my remaining block columns t
+    const T* ya = sw.bcast_y(st);
+    long b_ts = 0;
+    const T* gb = sw.route_g(st, &b_ts);
+    const int lj0 = st.lj0, ncols = st.lj1 - st.lj0;
     // (5) Y_t <- Y_t - Y_k G(t,k)^H for all my remaining block columns: one launch
     if (ncols > 0) {
       GemmArgsT<T> u{};
@@ -346,12 +110,12 @@ long triangular_solve_device(const TrsmProblem& p, double alpha_re, double alpha
           int* flag = oz_flag + step;
           oz_a.split(ya, ldy, ldy, s, 0, 0, flag);
           const bool strided = (pattern_n && Pe == 1);
-          const long nb_rows = strided ? static_cast<long>(li1 - li0) * nbp : static_cast<long>(ncols) * nbp;
-          oz_b.split(strided ? panelR : gb, nbp, nb_rows, s, nbp, static_cast<long>(tsz), flag);
-          const long b_row = strided ? (static_cast<long>(lj0) * Qe + ecol - (forward ? k + 1 : 0)) * nbp : 0;
+          const long nb_rows = strided ? static_cast<long>(st.li1 - st.li0) * nbp : static_cast<long>(ncols) * nbp;
+          oz_b.split(strided ? sw.panelR : gb, nbp, nb_rows, s, nbp, static_cast<long>(tsz), flag);
+          const long b_row = strided ? sw.panel_r_offset(st) * nbp : 0;
           launch_gemm_ozaki_i8(u, oz_a, 0, oz_b, b_row, s, strided ? static_cast<long>(Qe) * nbp : 0, flag);
           launch_gemm_nt_f64_if(u, flag, s);
-          launches += 4;
+          sw.launches += 4;
           done = true;
         }
       }
@@ -367,21 +131,9 @@ long triangular_solve_device(const TrsmProblem& p, double alpha_re, double alpha
       pool_free(oz_flag);
     }
   }
-  if (ltcY > 0) {
-    dim3 grid(static_cast<unsigned>(ltcY * nbp), static_cast<unsigned>((ldy + 1023) / 1024 > 0 ? (ldy + 1023) / 1024 : 1));
-    trsm_convert_y_kernel<T, false><<<grid, 256, 0, s>>>(b_user, ldb, lrb, lcb, y, ldy, ba, nbp, left, 1.0, 0.0);
-    DLAF_CUDA_CHECK(cudaGetLastError());
-    ++launches;
-  }
-  DLAF_CUDA_CHECK(cudaStreamSynchronize(s));
-  pool_free(a_slab);
-  pool_free(y);
-  pool_free(dloc);
-  pool_free(dbuf);
-  pool_free(panelY);
-  pool_free(panelR);
-  pool_free(panelG);
-  return launches;
+  sw.convert(false);
+  sw.release();
+  return sw.launches;
 }
 
 #define INST(T)                                                                                                              \

@@ -30,6 +30,20 @@ DLAF_EXTERN_C int dlaf_b200_triangular_solver_s(int ctx, char side, char uplo, c
 DLAF_EXTERN_C int dlaf_b200_triangular_solver_d(int ctx, char side, char uplo, char op, char diag, const double* alpha, const double* a, struct DLAF_descriptor desca, double* b, struct DLAF_descriptor descb) DLAF_NOEXCEPT;
 DLAF_EXTERN_C int dlaf_b200_triangular_solver_c(int ctx, char side, char uplo, char op, char diag, const dlaf_complex_c* alpha, const dlaf_complex_c* a, struct DLAF_descriptor desca, dlaf_complex_c* b, struct DLAF_descriptor descb) DLAF_NOEXCEPT;
 DLAF_EXTERN_C int dlaf_b200_triangular_solver_z(int ctx, char side, char uplo, char op, char diag, const dlaf_complex_z* alpha, const dlaf_complex_z* a, struct DLAF_descriptor desca, dlaf_complex_z* b, struct DLAF_descriptor descb) DLAF_NOEXCEPT;
+/* dlaf::triangular_multiplication (include/dlaf/multiplication/triangular.h:47-185; the reference has no C entry for it):
+ *   B <- alpha op(A) B  (side 'L')   or   B <- alpha B op(A)  (side 'R')
+ * for a triangular A (uplo 'L' / 'U', diag 'N' / 'U', op 'N' / 'T' / 'C'; all combinations, also on a P x Q grid) with the
+ * arguments, preconditions and local parts of dlaf_b200_triangular_solver_*: HOST local parts, b overwritten with the
+ * product, synchronous. alpha == 0 sets B to zero; an empty B is left alone. Returns 0. The _device flavour takes DEVICE
+ * local parts (the C++ surface's Backend::GPU / Device::GPU flavour) and is synchronous on cuda_stream. */
+DLAF_EXTERN_C int dlaf_b200_triangular_multiplication_s(int ctx, char side, char uplo, char op, char diag, const float* alpha, const float* a, struct DLAF_descriptor desca, float* b, struct DLAF_descriptor descb) DLAF_NOEXCEPT;
+DLAF_EXTERN_C int dlaf_b200_triangular_multiplication_d(int ctx, char side, char uplo, char op, char diag, const double* alpha, const double* a, struct DLAF_descriptor desca, double* b, struct DLAF_descriptor descb) DLAF_NOEXCEPT;
+DLAF_EXTERN_C int dlaf_b200_triangular_multiplication_c(int ctx, char side, char uplo, char op, char diag, const dlaf_complex_c* alpha, const dlaf_complex_c* a, struct DLAF_descriptor desca, dlaf_complex_c* b, struct DLAF_descriptor descb) DLAF_NOEXCEPT;
+DLAF_EXTERN_C int dlaf_b200_triangular_multiplication_z(int ctx, char side, char uplo, char op, char diag, const dlaf_complex_z* alpha, const dlaf_complex_z* a, struct DLAF_descriptor desca, dlaf_complex_z* b, struct DLAF_descriptor descb) DLAF_NOEXCEPT;
+DLAF_EXTERN_C int dlaf_b200_triangular_multiplication_device_s(int ctx, char side, char uplo, char op, char diag, const float* alpha, const float* a_dev, struct DLAF_descriptor desca, float* b_dev, struct DLAF_descriptor descb, void* cuda_stream) DLAF_NOEXCEPT;
+DLAF_EXTERN_C int dlaf_b200_triangular_multiplication_device_d(int ctx, char side, char uplo, char op, char diag, const double* alpha, const double* a_dev, struct DLAF_descriptor desca, double* b_dev, struct DLAF_descriptor descb, void* cuda_stream) DLAF_NOEXCEPT;
+DLAF_EXTERN_C int dlaf_b200_triangular_multiplication_device_c(int ctx, char side, char uplo, char op, char diag, const dlaf_complex_c* alpha, const dlaf_complex_c* a_dev, struct DLAF_descriptor desca, dlaf_complex_c* b_dev, struct DLAF_descriptor descb, void* cuda_stream) DLAF_NOEXCEPT;
+DLAF_EXTERN_C int dlaf_b200_triangular_multiplication_device_z(int ctx, char side, char uplo, char op, char diag, const dlaf_complex_z* alpha, const dlaf_complex_z* a_dev, struct DLAF_descriptor desca, dlaf_complex_z* b_dev, struct DLAF_descriptor descb, void* cuda_stream) DLAF_NOEXCEPT;
 /* dlaf::triangular_inverse (include/dlaf/inverse/triangular.h:38-76; the reference has no C entry for it): the `uplo`
  * triangle of the HOST local part a (diag 'U': its diagonal is assumed to be 1 and is neither read nor written) is
  * overwritten with the inverse of that triangular matrix. Collective over the grid of ctx, synchronous. Returns 0. */
@@ -62,12 +76,12 @@ DLAF_EXTERN_C int dlaf_b200_generalized_to_standard_device_s(int ctx, char uplo,
 DLAF_EXTERN_C int dlaf_b200_generalized_to_standard_device_d(int ctx, char uplo, double* a_dev, struct DLAF_descriptor desca, const double* b_dev, struct DLAF_descriptor descb, void* cuda_stream) DLAF_NOEXCEPT;
 DLAF_EXTERN_C int dlaf_b200_generalized_to_standard_device_c(int ctx, char uplo, dlaf_complex_c* a_dev, struct DLAF_descriptor desca, const dlaf_complex_c* b_dev, struct DLAF_descriptor descb, void* cuda_stream) DLAF_NOEXCEPT;
 DLAF_EXTERN_C int dlaf_b200_generalized_to_standard_device_z(int ctx, char uplo, dlaf_complex_z* a_dev, struct DLAF_descriptor desca, const dlaf_complex_z* b_dev, struct DLAF_descriptor descb, void* cuda_stream) DLAF_NOEXCEPT;
-/* fp64: number of steps of the last inverse / generalized_to_standard on ctx whose update ran on the native fp64 kernel because the int8 digit
- * guard fired (see dlaf_b200_guard_fallback_steps). */
+/* fp64: number of steps of the last inverse / generalized_to_standard / triangular multiplication on ctx whose update ran on the
+ * native fp64 kernel because the int8 digit guard fired (see dlaf_b200_guard_fallback_steps). */
 DLAF_EXTERN_C int dlaf_b200_last_inverse_guard_steps(int ctx) DLAF_NOEXCEPT;
-/* Number of this library's kernel launches issued by the last triangular solve / inverse on ctx. */
+/* Number of this library's kernel launches issued by the last triangular solve / multiplication / inverse on ctx. */
 DLAF_EXTERN_C long dlaf_b200_last_solver_launch_count(int ctx) DLAF_NOEXCEPT;
-/* Device time [ms] of the last triangular solve / inverse on ctx (CUDA events around the device-resident part: layout conversion,
+/* Device time [ms] of the last triangular solve / multiplication / inverse on ctx (CUDA events around the device-resident part: layout conversion,
  * diagonal-block inverses, the sweep; host <-> device copies excluded). */
 DLAF_EXTERN_C double dlaf_b200_last_solver_device_ms(int ctx) DLAF_NOEXCEPT;
 
